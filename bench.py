@@ -12,6 +12,7 @@ on the data path; configs[3] = 512 pages on 8 GPUs).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference            # the HF/PyTorch CPU path (oracle port) on the host cores
+    python bench.py --gpus 1 --steps 3 --warmup 3 --dump-outputs DIR    # also write the last timed step's outputs to DIR
 
 Prints ONE JSON line (rank 0).
 """
@@ -22,6 +23,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -31,6 +33,8 @@ sys.path.insert(0, ROOT)
 PAGE_HW = (1024, 1024)
 TEXT_TOKENS = 256
 METRIC = "pages/sec (1024x1024 doc images, greedy)"
+NCCL_LOG_PREFIX = os.path.join(tempfile.gettempdir(), "dots_ocr_b200_nccl_debug.")
+DUMP_BYTES = 64 << 20           # --dump-outputs: at most this much in all, half for the sequences, half for the embedding sample
 
 
 def _peaks():
@@ -216,6 +220,25 @@ def ids_checksum(new_ids) -> str:
     return f"{h:016x}"
 
 
+def dump_outputs(out, dump_dir: str) -> dict:
+    """Write what one generate() call returned under `dump_dir`: sequences.npy [B, T + N] (prompt + generated ids, exact in
+    float64), image_embeds.npy (float32, a sample of rows drawn with a fixed seed) and image_embeds_rows.npy (their indices).
+    The sample depends on the shape alone, so two builds run with the same arguments can be compared array for array."""
+    import numpy as np
+    import torch
+    seq = out.sequences.cpu().numpy().astype(np.float64)
+    assert seq.nbytes <= DUMP_BYTES // 2, f"sequences are {seq.nbytes} bytes: too large to dump"
+    emb = out.image_embeds
+    n, h = emb.shape
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(2718))[:min(n, (DUMP_BYTES // 2) // (4 * h + 8))].sort().values
+    arrays = {"sequences": seq, "image_embeds": emb[rows.to(emb.device)].float().cpu().numpy(),
+              "image_embeds_rows": rows.numpy().astype(np.float64)}
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dump_dir, f"{name}.npy"), a)
+    return {"dir": dump_dir, "shapes": {name: list(a.shape) for name, a in arrays.items()}}
+
+
 def make_workload(cfg, batch: int, rank: int, dev):
     """The benchmark's synthetic pages and prompts (shared with the parity test of this exact workload): pixel_values ~ N(0, 1)
     drawn on the device with seed 1234 + rank, prompts = 128 text ids + image pads + 128 text ids (seed 7)."""
@@ -257,8 +280,7 @@ def run_gpu(args):
         # NCCL_DEBUG is left as the caller set it; its output is routed to a file (NCCL_DEBUG_FILE, one per process) unless the caller
         # chose one, because NCCL keeps logging at process exit and the JSON must stay the LAST line of stdout
         if os.environ.get("NCCL_DEBUG") and not os.environ.get("NCCL_DEBUG_FILE"):
-            os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-            os.environ["NCCL_DEBUG_FILE"] = os.path.join(ROOT, "gpurun_out", "nccl_debug.%h.%p.log")
+            os.environ["NCCL_DEBUG_FILE"] = NCCL_LOG_PREFIX + "%h.%p.log"
         dist.init_process_group("nccl", device_id=dev)
 
     from dots_ocr_b200 import config, weights, ops
@@ -316,7 +338,7 @@ def run_gpu(args):
 
     per_step = {}
 
-    def timed(fn, k):
+    def timed(fn, k, name=None):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
@@ -329,7 +351,7 @@ def run_gpu(args):
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
         # per-step times of this rank (diagnostic only: the reported number is the whole region, max over ranks)
-        per_step[fn.__name__] = [round(a.elapsed_time(b), 1) for a, b in zip([e0] + marks[:-1], marks)]
+        per_step[name or fn.__name__] = [round(a.elapsed_time(b), 1) for a, b in zip([e0] + marks[:-1], marks)]
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
@@ -348,6 +370,7 @@ def run_gpu(args):
     dec_log = list(eng.decode_log)
     new_ids = last["out"].sequences[:, ids_dev.shape[1]:]
     checksum = ids_checksum(new_ids)
+    dumped = dump_outputs(last["out"], args.dump_outputs) if args.dump_outputs and rank == 0 else None
     # ---- timed region 2 (`e2e`): the public call with pinned host buffers, H2D and D2H inside
     ms_e2e = None
     if not args.no_e2e:
@@ -361,7 +384,7 @@ def run_gpu(args):
     clocks = sampler.stop() if rank == 0 else None
     # ---- separate pass: CUDA events around every prefill-side launch (kernel classes and their share of a step)
     ops.PROFILE = prof = []
-    ms_prof = timed(step_device, 1)
+    ms_prof = timed(step_device, 1, "instrumented_step")
     ops.PROFILE = None
 
     pages = B * world * args.steps
@@ -446,12 +469,14 @@ def run_gpu(args):
                           "instrumented_step": round(ms_prof, 2), "per_step_rank0": per_step},
             "kernels": by_kernel, "ids_checksum": {"value": checksum, "golden": golden, "matches_golden": (checksum == golden) if golden else None},
             "cpu_baseline": cpu}
+    if dumped:
+        line["outputs_dumped"] = dumped
     if world > 1:
         # NCCL's log of this run (routed to files above) is echoed on STDERR so that whoever reads the run's output still sees the
         # communicator's rank count; stdout carries nothing after the JSON line
-        if str(os.environ.get("NCCL_DEBUG_FILE", "")).startswith(os.path.join(ROOT, "gpurun_out", "nccl_debug.")):
+        if str(os.environ.get("NCCL_DEBUG_FILE", "")).startswith(NCCL_LOG_PREFIX):
             import glob
-            for f in sorted(glob.glob(os.path.join(ROOT, "gpurun_out", f"nccl_debug.*.{os.getpid()}.log"))):
+            for f in sorted(glob.glob(f"{NCCL_LOG_PREFIX}*.{os.getpid()}.log")):
                 try:
                     with open(f) as fh:
                         sys.stderr.write(fh.read())
@@ -481,7 +506,13 @@ def main():
                     help="decode layer variant (default: the engine default); see Engine.decode_mode")
     ap.add_argument("--attn-splits", dest="attn_splits", type=int, default=0, help="force the key-split count of the decode attention")
     ap.add_argument("--attn-impl", dest="attn_impl", default=None, choices=["tc", "mma"])
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0's pages) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path")
     global PAGE_HW
     PAGE_HW = (args.page, args.page)
     if args.impl == "reference":

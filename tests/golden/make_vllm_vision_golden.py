@@ -14,7 +14,9 @@ How the CUDA build of vLLM is made to run its model code on a GPU-less box (noth
     (dots_ocr.py:359-362).
 RMSNorm runs vLLM's native implementation, attention its torch-SDPA path, rotary its native apply.
 
-Outputs per case: the patch-embed output, every block's output, and the merged image embeddings.
+Outputs per case: the patch-embed output, every block's output, and the merged image embeddings.  The merged embeddings are
+stored whole; each per-layer output keeps a seeded sample of TAP_KEEP of its rows, with their indices under ``<name>_rows``,
+so that the file stays below 1 MB.
 """
 import os
 import sys
@@ -31,6 +33,15 @@ CASES = {                       # name -> image grids (t, h, w) in 14-px patches
 }
 SEED_W, SEED_X = 0, 3
 WIDE_GRIDS = [(1, 4, 6), (1, 2, 2)]      # full-width case: 1536 wide, 12 heads x 128, SwiGLU 4224, two blocks
+TAP_KEEP, SEED_ROWS = 0.25, 17
+
+
+def sample_rows(out, name, t):
+    """Store a seeded, sorted sample of the rows of the per-layer output `t` as `name`, and their indices as `name`_rows."""
+    t = t.reshape(-1, t.shape[-1]).numpy().astype(np.float32)
+    n = t.shape[0]
+    rows = np.sort(np.random.default_rng([SEED_ROWS, n, t.shape[1]]).choice(n, max(1, round(n * TAP_KEEP)), replace=False))
+    out[name], out[f"{name}_rows"] = t[rows], rows.astype(np.int64)
 
 
 def wide_config():
@@ -126,7 +137,7 @@ def main():
         out[f"{name}_grid"] = grid.numpy()
         out[f"{name}_image_embeds"] = y.numpy().astype(np.float32)
         for k, t in taps.items():
-            out[f"{name}_{k}"] = t.reshape(-1, t.shape[-1]).numpy().astype(np.float32)
+            sample_rows(out, f"{name}_{k}", t)
     # full-width case: a second tower object under the same vLLM context
     wcfg = wide_config()
     wck = vision_only_checkpoint(wcfg, SEED_W + 1)
@@ -135,7 +146,7 @@ def main():
     y, taps = run_tower(wide, pv, grid)
     out["wide_grid"] = grid.numpy()
     out["wide_image_embeds"] = y.numpy().astype(np.float32)
-    out["wide_block_1"] = taps["block_1"].reshape(-1, taps["block_1"].shape[-1]).numpy().astype(np.float32)
+    sample_rows(out, "wide_block_1", taps["block_1"])
     ctx.__exit__(None, None, None)
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "vllm_vision_tiny.npz")
     np.savez_compressed(path, **out)

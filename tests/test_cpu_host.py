@@ -127,8 +127,8 @@ def test_oracle_matches_golden_vectors():
 
 def test_vision_oracle_matches_vllm_own_vision_tower():
     """oracle/vision.py against vectors produced by vLLM's DotsVisionTransformer itself, run on CPU in fp32 on the same
-    seeded weights and inputs (tests/golden/make_vllm_vision_golden.py): patch embed, every block, merged embeddings.
-    fp32 both sides, so only summation order differs: 2e-5 of the tensor's range."""
+    seeded weights and inputs (tests/golden/make_vllm_vision_golden.py): patch embed, every block (on the stored sample of
+    rows), merged embeddings.  fp32 both sides, so only summation order differs: 2e-5 of the tensor's range."""
     from dots_ocr_b200 import config, weights
     from oracle.vision import VisionOracle
     sys.path.insert(0, GOLD)
@@ -140,10 +140,10 @@ def test_vision_oracle_matches_vllm_own_vision_tower():
         pv, grid = G.case_inputs(cfg, grids)
         assert np.array_equal(d[f"{name}_grid"], grid.numpy())
         out, layers = o.forward(pv, grid, return_layers=True)
-        want = [d[f"{name}_patch_embed"]] + [d[f"{name}_block_{i}"] for i in range(cfg.vision.num_hidden_layers)]
+        want = [f"{name}_patch_embed"] + [f"{name}_block_{i}" for i in range(cfg.vision.num_hidden_layers)]
         assert len(layers) == len(want)
-        for i, (a, b) in enumerate(zip(layers, want)):
-            b = torch.from_numpy(b)
+        for i, (a, k) in enumerate(zip(layers, want)):
+            a, b = a[torch.from_numpy(d[f"{k}_rows"])], torch.from_numpy(d[k])
             assert a.shape == b.shape
             assert float((a - b).abs().max()) <= 2e-5 * float(b.abs().max()), (name, i)
         ref = torch.from_numpy(d[f"{name}_image_embeds"])
@@ -153,7 +153,7 @@ def test_vision_oracle_matches_vllm_own_vision_tower():
     ow = VisionOracle(wcfg.vision, G.vision_only_checkpoint(wcfg, G.SEED_W + 1), torch.float32, "cpu")
     pv, grid = G.case_inputs(wcfg, G.WIDE_GRIDS)
     out, layers = ow.forward(pv, grid, return_layers=True)
-    for a, b in ((layers[-1], d["wide_block_1"]), (out, d["wide_image_embeds"])):
+    for a, b in ((layers[-1][torch.from_numpy(d["wide_block_1_rows"])], d["wide_block_1"]), (out, d["wide_image_embeds"])):
         b = torch.from_numpy(b)
         assert a.shape == b.shape and float((a - b).abs().max()) <= 2e-5 * float(b.abs().max())
 
@@ -641,3 +641,26 @@ def test_bench_roofline_traffic_comes_from_the_committed_ncu_capture():
     assert isinstance(g["b64_n512_p1024_rank0"], str) and len(g["b64_n512_p1024_rank0"]) == 16
     ids = __import__("torch").arange(12).view(3, 4)
     assert bench.ids_checksum(ids) == bench.ids_checksum(ids.clone()) != bench.ids_checksum(ids + 1)
+
+
+def test_bench_dump_outputs_writes_float_arrays_within_budget(tmp_path):
+    """bench.py --dump-outputs: sequences whole and exact, the image embeddings as a seeded sample of rows that the same shape
+    always draws the same way, every array float32 or float64, 64 MB in all at the headline shape."""
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+    from dots_ocr_b200.engine import GenerateOutput
+    seqs = torch.randint(0, 151643, (64, 1625 + 512))
+    emb = torch.randn(64 * 1369, 1536).to(torch.bfloat16)
+    info = bench.dump_outputs(GenerateOutput(sequences=seqs, image_embeds=emb), str(tmp_path / "a"))
+    bench.dump_outputs(GenerateOutput(sequences=seqs, image_embeds=emb.clone()), str(tmp_path / "b"))
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["image_embeds.npy", "image_embeds_rows.npy", "sequences.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 << 20
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert np.array_equal(got["sequences"], seqs.numpy()) and info["shapes"]["sequences"] == [64, 2137]
+    rows = got["image_embeds_rows"].astype(np.int64)
+    assert 1000 < rows.size < emb.shape[0] and np.all(np.diff(rows) > 0)
+    assert np.array_equal(got["image_embeds"], emb.float().numpy()[rows])
+    for f in files:
+        assert np.array_equal(got[f[:-4]], np.load(tmp_path / "b" / f))

@@ -127,32 +127,21 @@ def test_parse_chat_request_units():
             parse_chat_request(body)
 
 
-def test_unmodified_reference_client_talks_to_the_endpoint(endpoint, monkeypatch):
-    """The reference's own ``inference_with_vllm`` (imported from /root/reference when that checkout exists in this
-    container; it never exists on the GPU box) pointed at this endpoint returns the runner's text."""
+def test_unmodified_reference_client_talks_to_the_endpoint(endpoint):
+    """The request the reference's own ``inference_with_vllm`` sends (recorded from an unmodified dots.ocr checkout by
+    tests/golden/make_reference_client_golden.py), replayed against this endpoint: the reply parses as the OpenAI client the
+    reference uses parses it, and its content is the runner's text."""
     import os
-    import sys
-    import types
-    if not os.path.isfile("/root/reference/dots_ocr/model/inference.py"):
-        pytest.skip("reference checkout not present")
-    monkeypatch.syspath_prepend("/root/reference")
-    if "fitz" not in sys.modules:
-        monkeypatch.setitem(sys.modules, "fitz", types.ModuleType("fitz"))      # PyMuPDF is not installed; unused on this path
-    for k in [k for k in sys.modules if k == "dots_ocr" or k.startswith("dots_ocr.")]:
-        monkeypatch.delitem(sys.modules, k)
-    try:
-        from dots_ocr.model.inference import inference_with_vllm as ref_client
-    except ImportError as e:
-        pytest.skip(f"reference client not importable here: {e}")
+    from openai.types.chat import ChatCompletion
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_client_request.json")) as f:
+        rec = json.load(f)
+    assert rec["method"] == "POST" and rec["content_type"] == "application/json"
     r, base = endpoint
-    port = int(base.rsplit(":", 1)[1])
-    img = Image.new("RGB", (64, 48), (200, 100, 50))
-    text = ref_client(img, "Parse this page", protocol="http", ip="127.0.0.1", port=port, max_completion_tokens=99,
-                      model_name="rednote-hilab/dots.mocr")
+    code, body = _post(base, rec["path"], rec["body"])
+    assert code == 200, body
+    text = ChatCompletion.model_validate(body).choices[0].message.content
     assert text == '[{"bbox": [0, 0, 64, 48], "category": "Text", "text": "Parse th"}]'
     assert r.calls == [((64, 48), (200, 100, 50), "Parse this page", 99)]
-    for k in [k for k in sys.modules if k == "dots_ocr" or k.startswith("dots_ocr.")]:
-        del sys.modules[k]
 
 
 def test_the_mirror_client_uses_http_on_a_machine_without_a_gpu(endpoint, monkeypatch, capsys):
@@ -178,7 +167,8 @@ def test_the_mirror_client_uses_http_on_a_machine_without_a_gpu(endpoint, monkey
         from dots_ocr_b200 import DotsOCRParser
         p = DotsOCRParser(ip="127.0.0.1", port=port, max_completion_tokens=9)
         assert p._inference_with_vllm(img, "q").startswith('[{"bbox": [0, 0, 48, 32]') and r.calls[-1][2:] == ("q", 9)
-        # an installed runner wins over the transport arguments
+        # in the default transport mode an installed runner wins over the transport arguments
+        monkeypatch.delenv("DOTS_B200_TRANSPORT", raising=False)
         class Local:
             def infer(self, image, prompt, max_new_tokens=0):
                 return "local"

@@ -26,11 +26,12 @@ def test_engine_vision_tower_matches_vllm_vectors():
     for name, grids in G.CASES.items():
         pv, grid = G.case_inputs(cfg, grids)
         out, layers = eng.encode_images(pv.to(DEV), grid, return_layers=True)
-        want = [d[f"{name}_patch_embed"]] + [d[f"{name}_block_{i}"] for i in range(cfg.vision.num_hidden_layers)]
+        want = [f"{name}_patch_embed"] + [f"{name}_block_{i}" for i in range(cfg.vision.num_hidden_layers)]
         assert len(layers) == len(want)
-        for i, (a, b) in enumerate(zip(layers, want)):
-            b = torch.from_numpy(b)
-            err = float((a.float().cpu() - b).abs().max() / b.abs().max())
+        for i, (a, k) in enumerate(zip(layers, want)):
+            a, b = a.float().cpu()[torch.from_numpy(d[f"{k}_rows"])], torch.from_numpy(d[k])
+            assert a.shape == b.shape
+            err = float((a - b).abs().max() / b.abs().max())
             assert err < TOL, (name, i, err)
         ref = torch.from_numpy(d[f"{name}_image_embeds"])
         err = float((out.float().cpu() - ref).abs().max() / ref.abs().max())
