@@ -55,18 +55,19 @@ class BatchingRunner:
         self._worker.start()
 
     # -- caller side ------------------------------------------------------------------------------------------------
-    def submit(self, image, prompt: str, max_new_tokens: int = 512) -> Future:
+    def submit(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> Future:
+        """sampling: None (greedy) or a ``SamplingParams``; a missing seed is drawn here, at submission."""
         if self._closed:
             raise RuntimeError("BatchingRunner is closed")
         fut: Future = Future()
-        self._q.put((image, prompt, int(max_new_tokens), fut))
+        self._q.put((image, prompt, int(max_new_tokens), fut, None if sampling is None else sampling.with_seed()))
         return fut
 
-    def infer(self, image, prompt: str, max_new_tokens: int = 512) -> str:
-        return self.submit(image, prompt, max_new_tokens).result()
+    def infer(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> str:
+        return self.submit(image, prompt, max_new_tokens, sampling).result()
 
-    def infer_batch(self, images, prompts, max_new_tokens: int = 512) -> List[str]:
-        futs = [self.submit(im, pr, max_new_tokens) for im, pr in zip(images, prompts)]
+    def infer_batch(self, images, prompts, max_new_tokens: int = 512, sampling=None) -> List[str]:
+        futs = [self.submit(im, pr, max_new_tokens, sampling) for im, pr in zip(images, prompts)]
         return [f.result() for f in futs]
 
     def close(self, timeout: Optional[float] = 5.0) -> None:
@@ -115,6 +116,10 @@ class BatchingRunner:
         self.batches.append(len(batch))
         try:
             kw = {"budgets": [b[2] for b in batch]} if self._takes_budgets else {}
+            if any(b[4] is not None for b in batch):
+                # per-row parameters; the pages that did not ask for sampling decode greedily beside the others
+                from .sampling import GREEDY
+                kw["sampling"] = [GREEDY if b[4] is None else b[4] for b in batch]
             texts = self.runner.infer_batch([b[0] for b in batch], [b[1] for b in batch], max_new_tokens=n_new, **kw)
         except Exception as e:          # noqa: BLE001 -- the error belongs to the callers, not to the worker thread
             if len(batch) == 1:

@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdots_ocr_b200.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["common.cu", "gemm_tcgen05.cu", "attn_fwd_mma.cu", "attn_fwd_tcgen05.cu", "attn_decode.cu", "decode_gemm.cu", "elementwise.cu", "partition.cu"]
+SOURCES = ["common.cu", "gemm_tcgen05.cu", "attn_fwd_mma.cu", "attn_fwd_tcgen05.cu", "attn_decode.cu", "decode_gemm.cu", "elementwise.cu", "sampling.cu", "partition.cu"]
 # documented negative results (DESIGN.md section 8): compiled into the library only on request, never by default
 EXPERIMENTS = ["experiments/attn_fwd_tcgen05_pair.cu", "experiments/decode_chain.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -5,7 +5,7 @@ that stops after 300 tokens idles while its neighbour writes 4000, and pages tha
 Here the decode state is a fixed set of SLOTS (rows of one KV cache / one captured decode graph).  The scheduler alternates
 
     admit    free slots <- queued pages: ViT + prefill write the new rows of the cache, first token selected
-    decode   ``chunk`` greedy steps for every slot (one graph replay per step)
+    decode   ``chunk`` steps for every slot (one graph replay per step)
     harvest  rows that produced a stop id or used up their own token budget are answered and their slots freed
 
 so a finished row is refilled at the next chunk boundary while the other rows keep their context.  No kernel knows about
@@ -63,25 +63,42 @@ class EngineSlots:
         self._warm = False
 
     # -- admission ------------------------------------------------------------------------------------------------------
-    def prepare(self, image, prompt: str):
-        """Host half of admission (runs in the scheduler thread before the GPU is touched): uint8 page + prompt ids."""
+    def prepare(self, image, prompt: str, sampling=None):
+        """Host half of admission (runs in the scheduler thread before the GPU is touched): uint8 page + prompt ids +
+        the page's sampling parameters (None: greedy)."""
         from .processing import page_to_u8, model_image_tokens
         page = page_to_u8(image)                               # original size: the resize runs on the GPU at admission
         n_img = model_image_tokens(int(page.shape[0]), int(page.shape[1]), self.min_pixels, self.max_pixels)
         ids = self.tokenizer.encode_chat(prompt, n_img)
         if len(ids) > self.max_prompt:
             raise ValueError(f"prompt of {len(ids)} tokens exceeds the session's max_prompt {self.max_prompt}")
-        return page, ids
+        return page, ids, sampling
+
+    def _enable_sampling(self) -> None:
+        """First sampled page of the session: add the per-row parameter arrays (every row greedy until admitted with
+        parameters) and drop the captured graph, so that the next step captures it with dots_sample_advance.  A session
+        that only ever sees greedy pages keeps the greedy kernel."""
+        import torch
+        st, n, dev = self.st, self.n_slots, self.engine.device
+        st["temperature"] = torch.zeros(n, device=dev, dtype=torch.float32)
+        st["top_p"] = torch.ones(n, device=dev, dtype=torch.float32)
+        st["top_k"] = torch.zeros(n, device=dev, dtype=torch.int32)
+        st["seed"] = torch.zeros(n, device=dev, dtype=torch.int64)
+        self._graph = None
 
     def admit(self, slots: Sequence[int], prepared: Sequence) -> None:
         """ViT + prefill of the new pages into cache rows ``slots``; selects each row's first token."""
         import torch
         from . import ops
+        from .sampling import GREEDY, host_arrays
         eng, st, dev = self.engine, self.st, self.engine.device
         t = eng.cfg.text
+        params = [item[2] if len(item) > 2 else None for item in prepared]
+        if "temperature" not in st and any(p is not None for p in params):
+            self._enable_sampling()
         with torch.no_grad(), torch.cuda.device(dev):
-            pages = [p.to(dev, non_blocking=True) for p, _ in prepared]
-            rows = [ids for _, ids in prepared]
+            pages = [item[0].to(dev, non_blocking=True) for item in prepared]
+            rows = [item[1] for item in prepared]
             seq_lens = [len(r) for r in rows]
             ids_packed = torch.tensor([i for r in rows for i in r], dtype=torch.int64, device=dev)
             positions = torch.cat([torch.arange(n, dtype=torch.int32) for n in seq_lens]).to(dev)
@@ -106,9 +123,15 @@ class EngineSlots:
             pos = (lens - 1).to(torch.int32)
             ctx = lens.to(torch.int32)
             fin = torch.zeros(n, dtype=torch.int32, device=dev)
-            ops.argmax_advance(logits, last, out, step, pos, ctx, fin, tuple(self.stops[: ops.MAX_STOP_IDS]), self.pad, None)
-            eng.launches += 5
             idx = torch.tensor(list(slots), dtype=torch.int64, device=dev)
+            if "temperature" in st:
+                arrs = [a.to(dev) for a in host_arrays([GREEDY if p is None else p.with_seed() for p in params])]
+                ops.sample_advance(logits, last, *arrs, out, step, pos, ctx, fin, tuple(self.stops[: ops.MAX_STOP_IDS]), self.pad, None)
+                for name, a in zip(("temperature", "top_p", "top_k", "seed"), arrs):
+                    st[name].index_copy_(0, idx, a)
+            else:
+                ops.argmax_advance(logits, last, out, step, pos, ctx, fin, tuple(self.stops[: ops.MAX_STOP_IDS]), self.pad, None)
+            eng.launches += 5
             st["last"].index_copy_(0, idx, last)
             st["out_ids"].index_copy_(0, idx, out)
             st["step"].index_copy_(0, idx, step)
@@ -118,7 +141,7 @@ class EngineSlots:
 
     # -- decode ---------------------------------------------------------------------------------------------------------
     def step(self, k: int) -> None:
-        """``k`` greedy steps for every slot (idle rows run along on a pad token)."""
+        """``k`` decode steps for every slot (idle rows run along on a pad token)."""
         import torch
         from . import ops
         eng, st = self.engine, self.st
@@ -149,7 +172,8 @@ class EngineSlots:
         return self.st["out_ids"][slot, :n].tolist()
 
     def rearm(self, slots: Sequence[int]) -> None:
-        """Park rows: finished, at position 0 with one visible key, so that running along stays inside their cache row."""
+        """Park rows: finished, at position 0 with one visible key, so that running along stays inside their cache row;
+        greedy, so that a parked row costs the sampling kernel its argmax pass only."""
         import torch
         if not slots:
             return
@@ -160,6 +184,8 @@ class EngineSlots:
         st["pos"].index_fill_(0, idx, 0)
         st["ctx_len"].index_fill_(0, idx, 1)
         st["last"].index_fill_(0, idx, self.pad)
+        if "temperature" in st:
+            st["temperature"].index_fill_(0, idx, 0.0)
 
     def decode_text(self, ids: List[int]) -> str:
         return self.tokenizer.decode(ids)
@@ -169,10 +195,11 @@ class EngineSlots:
 # scheduler
 # =====================================================================================================================
 class _Req:
-    __slots__ = ("image", "prompt", "budget", "future", "tokens", "arrived")
+    __slots__ = ("image", "prompt", "budget", "future", "tokens", "arrived", "sampling")
 
-    def __init__(self, image, prompt, budget, future, tokens):
+    def __init__(self, image, prompt, budget, future, tokens, sampling=None):
         self.image, self.prompt, self.budget, self.future, self.tokens = image, prompt, budget, future, tokens
+        self.sampling = sampling                   # SamplingParams with its seed, or None (greedy)
         self.arrived = time.monotonic()
 
 
@@ -198,19 +225,20 @@ class ContinuousBatcher:
         self._worker.start()
 
     # -- caller side ------------------------------------------------------------------------------------------------
-    def submit(self, image, prompt: str, max_new_tokens: int = 512) -> Future:
+    def submit(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> Future:
+        """sampling: None (greedy) or a ``SamplingParams``; a missing seed is drawn here, at submission."""
         if self._closed:
             raise RuntimeError("ContinuousBatcher is closed")
         fut: Future = Future()
         budget = max(1, min(int(max_new_tokens), int(self.backend.max_new)))
-        self._q.put(_Req(image, prompt, budget, fut, max(1, page_vit_tokens(image))))
+        self._q.put(_Req(image, prompt, budget, fut, max(1, page_vit_tokens(image)), None if sampling is None else sampling.with_seed()))
         return fut
 
-    def infer(self, image, prompt: str, max_new_tokens: int = 512) -> str:
-        return self.submit(image, prompt, max_new_tokens).result()
+    def infer(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> str:
+        return self.submit(image, prompt, max_new_tokens, sampling).result()
 
-    def infer_batch(self, images, prompts, max_new_tokens: int = 512) -> List[str]:
-        futs = [self.submit(im, pr, max_new_tokens) for im, pr in zip(images, prompts)]
+    def infer_batch(self, images, prompts, max_new_tokens: int = 512, sampling=None) -> List[str]:
+        futs = [self.submit(im, pr, max_new_tokens, sampling) for im, pr in zip(images, prompts)]
         return [f.result() for f in futs]
 
     def close(self, timeout: Optional[float] = 30.0) -> None:
@@ -252,7 +280,7 @@ class ContinuousBatcher:
         ready, slots = [], []
         for r in picked:
             try:
-                ready.append((r, b.prepare(r.image, r.prompt)))
+                ready.append((r, b.prepare(r.image, r.prompt) if r.sampling is None else b.prepare(r.image, r.prompt, sampling=r.sampling)))
             except Exception as e:      # noqa: BLE001 -- this page's caller gets the error; the others go on
                 r.future.set_exception(e)
         if ready:

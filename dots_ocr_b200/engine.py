@@ -355,7 +355,7 @@ class Engine:
         )
 
     def _decode_step(self, st: dict):
-        """One greedy step for the whole batch; every call is a C-ABI kernel launch (graph-capturable)."""
+        """One decode step for the whole batch; every call is a C-ABI kernel launch (graph-capturable)."""
         t = self.cfg.text
         nq, nkv, hd = t.num_attention_heads, t.num_key_value_heads, t.head_dim
         H, I = t.hidden_size, t.intermediate_size
@@ -407,12 +407,23 @@ class Engine:
                 ops.gemm_skinny(st["act"], L["down"], pl["down"], partial=st["partial"])
                 ops.decode_residual_rmsnorm(st["partial"], pl["down"], st["resid"], nxt, st["normed"], t.rms_norm_eps)
             ops.gemm_skinny(st["normed"], self.lm_head, 1, out_bf16=st["logits"])
-        ops.argmax_advance(st["logits"], st["last"], st["out_ids"], st["step"], st["pos"], st["ctx_len"], st["finished"],
-                           st["stops"], st["pad"], st["forced"])
+        self._select(st)
+
+    @staticmethod
+    def _select(st: dict) -> None:
+        """Token selection + bookkeeping of one step: the sampling kernel when the state carries per-row sampling
+        parameters, else the greedy argmax kernel."""
+        if "temperature" in st:
+            ops.sample_advance(st["logits"], st["last"], st["temperature"], st["top_p"], st["top_k"], st["seed"], st["out_ids"], st["step"],
+                               st["pos"], st["ctx_len"], st["finished"], st["stops"], st["pad"], st["forced"])
+        else:
+            ops.argmax_advance(st["logits"], st["last"], st["out_ids"], st["step"], st["pos"], st["ctx_len"], st["finished"],
+                               st["stops"], st["pad"], st["forced"])
 
     def _new_decode_state(self, B: int, lens: torch.Tensor, kc, vc, ctx_max: int, N: int, eos_token_id=None, pad_token_id: int = 0,
-                          forced_ids: Optional[torch.Tensor] = None) -> dict:
-        """Every buffer one decode step touches (allocated once per generate; the CUDA graph captures their addresses)."""
+                          forced_ids: Optional[torch.Tensor] = None, sampling: bool = False) -> dict:
+        """Every buffer one decode step touches (allocated once per generate; the CUDA graph captures their addresses).
+        ``sampling``: also the per-row parameter arrays of ``dots_sample_advance`` (the values are written per call)."""
         t = self.cfg.text
         dev = self.device
         H = t.hidden_size
@@ -443,6 +454,11 @@ class Engine:
             st["normed_t"], st["attn_t"], st["act_t"] = tiled(H), tiled(t.num_attention_heads * t.head_dim), tiled(t.intermediate_size)
         st["stats"] = torch.zeros((2, -(-H // 128) * 64), device=dev, dtype=torch.float32)
         st["counters"] = torch.zeros(2 * t.num_hidden_layers, device=dev, dtype=torch.int32)
+        if sampling:
+            st["temperature"] = torch.zeros(B, device=dev, dtype=torch.float32)
+            st["top_p"] = torch.ones(B, device=dev, dtype=torch.float32)
+            st["top_k"] = torch.zeros(B, device=dev, dtype=torch.int32)
+            st["seed"] = torch.zeros(B, device=dev, dtype=torch.int64)
         return st
 
     def decode_weight_bytes(self) -> int:
@@ -475,13 +491,20 @@ class Engine:
                  pixel_values: Optional[torch.Tensor] = None, image_grid_thw=None, max_new_tokens: int = 16,
                  eos_token_id=None, pad_token_id: int = 0, forced_ids: Optional[torch.Tensor] = None,
                  return_logits: bool = False, use_graph: bool = True, image_embeds: Optional[torch.Tensor] = None,
-                 pages_u8=None, min_pixels: Optional[int] = None, max_pixels: Optional[int] = None, **unused) -> GenerateOutput:
-        """HF-shaped greedy generation: returns ids [B, T + N'] including the prompt (parser.py:110-113)."""
+                 pages_u8=None, min_pixels: Optional[int] = None, max_pixels: Optional[int] = None, sampling=None,
+                 **unused) -> GenerateOutput:
+        """HF-shaped generation: returns ids [B, T + N'] including the prompt (parser.py:110-113).  Greedy unless
+        ``sampling`` (one ``SamplingParams`` for every row, or a sequence of B) or HF's ``do_sample=True`` (with
+        ``temperature`` / ``top_p`` / ``top_k``, HF defaults 1.0 / 1.0 / 50) asks for sampling (dots_ocr_b200/sampling.py)."""
+        from . import sampling as _sampling
         t = self.cfg.text
         dev = self.device
         ids = input_ids.to(dev).long()
         B, Tpad = ids.shape
         assert B <= 256, "batch > 256 pages per call is not supported; shard the pages"
+        if sampling is None:
+            sampling = _sampling.from_hf_kwargs(unused)
+        rows = None if sampling is None else _sampling.per_row(sampling, B)
         mask = torch.ones_like(ids) if attention_mask is None else attention_mask.to(dev).long()
         lens = mask.sum(dim=1).to(torch.int64)
         seq_lens = lens.tolist()
@@ -512,12 +535,13 @@ class Engine:
         # KV cache, decode workspaces and the captured decode graph are kept from call to call when the shape key repeats
         # (a serving loop and the benchmark call generate with the same batch geometry over and over)
         stops_key = tuple(stop_list(eos_token_id)[: ops.MAX_STOP_IDS])
-        key = (B, ctx_max, N, stops_key, int(pad_token_id), self.decode_mode, self.attn_splits, ops.DECODE_CLUSTER, int(self.decode_sms))
+        key = (B, ctx_max, N, stops_key, int(pad_token_id), self.decode_mode, self.attn_splits, ops.DECODE_CLUSTER, int(self.decode_sms),
+               rows is not None)
         ent = self._dec_cache if (self._dec_cache is not None and self._dec_cache["key"] == key and forced_ids is None) else None
         if ent is None:
             self._dec_cache = None                      # release the previous geometry's buffers before allocating new ones
             kc, vc = self._alloc_cache(B, ctx_max)
-            st = self._new_decode_state(B, lens, kc, vc, ctx_max, N, eos_token_id, pad_token_id, forced_ids)
+            st = self._new_decode_state(B, lens, kc, vc, ctx_max, N, eos_token_id, pad_token_id, forced_ids, sampling=rows is not None)
             ent = dict(key=key, st=st, graph=None)
             if forced_ids is None:
                 self._dec_cache = ent
@@ -530,6 +554,9 @@ class Engine:
             st["finished"].zero_()
             st["pos"].copy_((lens - 1).to(torch.int32))
             st["ctx_len"].copy_(lens.to(torch.int32))
+        if rows is not None:
+            for name, v in zip(("temperature", "top_p", "top_k", "seed"), _sampling.host_arrays(rows)):
+                st[name].copy_(v)
         x = self._prefill(ids_packed, slots, image_embeds, cu, seq_lens, positions, seq_of_tok, kc, vc, ctx_max)
         pl = st["plan"]
         all_logits = torch.empty((N, B, t.vocab_size), device=dev, dtype=torch.bfloat16) if return_logits else None
@@ -539,8 +566,7 @@ class Engine:
         hl = ops.gather_rows(x, last_rows)
         ops.rmsnorm(hl, self.final_norm, t.rms_norm_eps, out=st["normed"])
         ops.gemm_skinny(st["normed"], self.lm_head, 1, out_bf16=st["logits"])
-        ops.argmax_advance(st["logits"], st["last"], st["out_ids"], st["step"], st["pos"], st["ctx_len"], st["finished"],
-                           st["stops"], st["pad"], st["forced"])
+        self._select(st)
         self.launches += 4
         del x
         if return_logits:

@@ -94,12 +94,17 @@ def inference_with_vllm(
         model_name="rednote-hilab/dots.mocr",
         system_prompt=None,
         ) -> Optional[str]:
-    """Greedy page inference.  ``temperature``/``top_p`` are accepted for signature compatibility; the
-    engine decodes greedily (BASELINE.json fixes greedy), which is the temperature -> 0 limit."""
+    """Page inference.  Over HTTP, ``temperature`` / ``top_p`` go to the server as the reference sends them.  In process
+    they are honoured under the sampling policy ``request`` (``DOTS_B200_SAMPLING=request``, dots_ocr_b200/sampling.py);
+    under the default ``greedy`` the engine decodes greedily (BASELINE.json fixes greedy), the temperature -> 0 limit."""
     if not _serve_in_process():
         return _http_chat(image, prompt, protocol, ip, port, temperature, top_p, max_completion_tokens, model_name, system_prompt)
+    from ..sampling import SamplingParams, sampling_policy
     runner = get_default_runner()
     text = prompt if system_prompt is None else f"{system_prompt}\n{prompt}"
+    if sampling_policy() == "request":
+        return runner.infer(image, text, max_new_tokens=max_completion_tokens,
+                            sampling=SamplingParams(temperature=float(temperature), top_p=float(top_p)))
     return runner.infer(image, text, max_new_tokens=max_completion_tokens)
 
 

@@ -34,7 +34,7 @@ class _Echo:
     def __init__(self, rank: int, delay: float, fail_on: str):
         self.rank, self.delay, self.fail_on = rank, delay, fail_on
 
-    def infer(self, image, prompt, max_new_tokens=512):
+    def infer(self, image, prompt, max_new_tokens=512, sampling=None):
         import time
         time.sleep(self.delay)
         if "die" in prompt:
@@ -42,7 +42,8 @@ class _Echo:
             os._exit(3)                                # a worker lost to a device fault
         if self.fail_on and self.fail_on in prompt:
             raise ValueError(f"worker {self.rank} refuses {prompt!r}")
-        return f"rank{self.rank}|{getattr(image, 'size', image)}|{prompt}|{max_new_tokens}"
+        out = f"rank{self.rank}|{getattr(image, 'size', image)}|{prompt}|{max_new_tokens}"
+        return out if sampling is None else f"{out}|{sampling!r}"
 
 
 def echo_worker(rank: int, delay: float = 0.0, fail_on: str = "", die_at_start: int = -1):
@@ -73,7 +74,7 @@ def _worker_main(rank: int, factory: Callable, factory_args: tuple, req_q, res_q
     if submit is None:
         from concurrent.futures import ThreadPoolExecutor
         pool = ThreadPoolExecutor(max_workers=64, thread_name_prefix=f"dots-w{rank}")
-        submit = lambda im, pr, n: pool.submit(runner.infer, im, pr, max_new_tokens=n)        # noqa: E731
+        submit = lambda im, pr, n, **kw: pool.submit(runner.infer, im, pr, max_new_tokens=n, **kw)        # noqa: E731
 
     def done(req_id, fut):
         e = fut.exception()
@@ -83,9 +84,10 @@ def _worker_main(rank: int, factory: Callable, factory_args: tuple, req_q, res_q
         item = req_q.get()
         if item is None:
             break
-        req_id, image, prompt, n_new = item
+        req_id, image, prompt, n_new, sampling = item
         try:
-            submit(image, prompt, n_new).add_done_callback(lambda f, r=req_id: done(r, f))
+            kw = {} if sampling is None else {"sampling": sampling}        # only a request that carries parameters passes them on
+            submit(image, prompt, n_new, **kw).add_done_callback(lambda f, r=req_id: done(r, f))
         except Exception as e:      # noqa: BLE001
             res_q.put((rank, req_id, False, _portable(e)))
     if pool is not None:
@@ -126,7 +128,8 @@ class MultiGpuRunner:
         self._collector.start()
 
     # -- caller side ------------------------------------------------------------------------------------------------
-    def submit(self, image, prompt: str, max_new_tokens: int = 512) -> Future:
+    def submit(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> Future:
+        """sampling: None (greedy) or a ``SamplingParams``; a missing seed is drawn here, in the front process."""
         if self._closed:
             raise RuntimeError("MultiGpuRunner is closed")
         weight = max(1, page_vit_tokens(image))
@@ -139,14 +142,14 @@ class MultiGpuRunner:
             rid = next(self._ids)
             self._pending[rid] = (fut, k, weight)
             self._load[k] += weight
-        self._reqs[k].put((rid, image, prompt, int(max_new_tokens)))
+        self._reqs[k].put((rid, image, prompt, int(max_new_tokens), None if sampling is None else sampling.with_seed()))
         return fut
 
-    def infer(self, image, prompt: str, max_new_tokens: int = 512) -> str:
-        return self.submit(image, prompt, max_new_tokens).result()
+    def infer(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> str:
+        return self.submit(image, prompt, max_new_tokens, sampling).result()
 
-    def infer_batch(self, images, prompts, max_new_tokens: int = 512) -> List[str]:
-        futs = [self.submit(im, pr, max_new_tokens) for im, pr in zip(images, prompts)]
+    def infer_batch(self, images, prompts, max_new_tokens: int = 512, sampling=None) -> List[str]:
+        futs = [self.submit(im, pr, max_new_tokens, sampling) for im, pr in zip(images, prompts)]
         return [f.result() for f in futs]
 
     def close(self, timeout: float = 10.0) -> None:

@@ -366,6 +366,31 @@ def argmax_advance(logits, next_ids, out_ids=None, step=None, pos=None, ctx_len=
     _lib.check(rc, "dots_argmax_advance")
 
 
+def sample_advance(logits, next_ids, temperature, top_p, top_k, seed, out_ids=None, step=None, pos=None, ctx_len=None,
+                   finished=None, stop_ids=(), pad_id: int = 0, forced_ids=None):
+    """``argmax_advance`` with a sampled token per row (DESIGN.md section 3): ``temperature`` / ``top_p`` float32 [B],
+    ``top_k`` int32 [B], ``seed`` int64 [B] (the bits of a u64) are device arrays read when the kernel runs, so a captured
+    graph follows later writes to them.  Rows with temperature < 1e-5 get exactly what ``argmax_advance`` gives them."""
+    _bf16_2d(logits, "logits")
+    B, V = logits.shape
+    for t, name, dt in ((temperature, "temperature", torch.float32), (top_p, "top_p", torch.float32),
+                        (top_k, "top_k", torch.int32), (seed, "seed", torch.int64)):
+        if not (t.is_cuda and t.dtype == dt and t.is_contiguous() and t.numel() == B):
+            raise ValueError(f"{name}: need a contiguous CUDA {dt} tensor of {B} elements, got {t.dtype} {tuple(t.shape)}")
+    if isinstance(stop_ids, int):
+        stop_ids = () if stop_ids < 0 else (stop_ids,)
+    stops = [int(s) for s in stop_ids]
+    if len(stops) > K["DOTS_MAX_STOP_IDS"]:
+        raise ValueError(f"at most {K['DOTS_MAX_STOP_IDS']} stop ids are handled on the device, got {len(stops)}")
+    arr = (_ll * max(1, len(stops)))(*stops)
+    rc = _lib.load().dots_sample_advance(_p(logits), _ll(logits.stride(0)), B, V, _p(next_ids), _p(out_ids),
+                                         _ll(out_ids.stride(0) if out_ids is not None else 0), _p(step), _p(pos), _p(ctx_len),
+                                         _p(finished), arr, len(stops), _ll(pad_id), _p(forced_ids),
+                                         _ll(forced_ids.stride(0) if forced_ids is not None else 0), _p(temperature), _p(top_p),
+                                         _p(top_k), _p(seed), _stream())
+    _lib.check(rc, "dots_sample_advance")
+
+
 def decode_embed_rmsnorm(ids, table, w, resid, normed, eps, counters=None, tile_rows: int = 0):
     """tile_rows > 0: ``normed`` is written k-block-tiled (the B operand of the cluster GEMMs), else row-major."""
     V, H = table.shape

@@ -73,6 +73,10 @@ class DotsOCRParser:
 
     def _inference_with_vllm(self, image, prompt):
         if self._runner is not None:
+            from .sampling import SamplingParams, sampling_policy
+            if sampling_policy() == "request":         # the parser's temperature / top_p, as the reference sends them to its server
+                return self._runner.infer(image, prompt, max_new_tokens=self.max_completion_tokens,
+                                          sampling=SamplingParams(temperature=float(self.temperature), top_p=float(self.top_p)))
             return self._runner.infer(image, prompt, max_new_tokens=self.max_completion_tokens)
         return inference_with_vllm(image, prompt, model_name=self.model_name, protocol=self.protocol, ip=self.ip,
                                    port=self.port, temperature=self.temperature, top_p=self.top_p,

@@ -58,8 +58,9 @@ class PageRunner:
         return cls(engine_factory(cfg, ckpt, device), tokenizer)
 
     def infer_batch(self, images: Sequence, prompts: Sequence[str], max_new_tokens: int = 512, gpu_preprocess: bool = True,
-                    budgets: Optional[Sequence[int]] = None) -> List[str]:
-        """gpu_preprocess: the whole image processor (resize, rescale / normalise / patchify) on the GPU (3 B per pixel over PCIe instead of
+                    budgets: Optional[Sequence[int]] = None, sampling=None) -> List[str]:
+        """sampling: None (greedy), one ``SamplingParams`` for every page or one per page (dots_ocr_b200/sampling.py).
+        gpu_preprocess: the whole image processor (resize, rescale / normalise / patchify) on the GPU (3 B per pixel over PCIe instead of
         12); False = the reference's host processor output (fp32 pixel_values) as `generate` input."""
         n_new = max(1, min(int(max_new_tokens), self.cap))
         if gpu_preprocess:
@@ -77,6 +78,8 @@ class PageRunner:
                 dict(pixel_values=inputs["pixel_values"].to(dev), image_grid_thw=inputs["image_grid_thw"])
             # every stop id of the checkpoint's generation config when the tokenizer knows them (HF accepts a list too)
             stops = list(getattr(self.tokenizer, "stop_ids", ())) or self.tokenizer.eos_token_id
+            if sampling is not None:
+                kw["sampling"] = sampling
             out = self.engine.generate(input_ids=inputs["input_ids"].to(dev), attention_mask=inputs["attention_mask"].to(dev),
                                        max_new_tokens=n_new, eos_token_id=stops,
                                        pad_token_id=self.tokenizer.pad_token_id, **kw)
@@ -86,5 +89,5 @@ class PageRunner:
         lim = [n_new] * len(seq) if budgets is None else [max(1, min(int(b), n_new)) for b in budgets]
         return [self.tokenizer.decode(row[T:T + k].tolist()) for row, k in zip(seq, lim)]
 
-    def infer(self, image, prompt: str, max_new_tokens: int = 512) -> str:
-        return self.infer_batch([image], [prompt], max_new_tokens)[0]
+    def infer(self, image, prompt: str, max_new_tokens: int = 512, sampling=None) -> str:
+        return self.infer_batch([image], [prompt], max_new_tokens, sampling=sampling)[0]

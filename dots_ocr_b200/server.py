@@ -11,8 +11,15 @@ point ``--ip/--port`` at a B200 box:
 Only what that client needs is here: ``POST /v1/chat/completions`` (non-streaming), ``GET /v1/models``, ``GET /health``.
 Request threads block on the process-wide request front (``dots_ocr_b200/continuous.py:serving_front``: continuous batching by
 default, ``DOTS_B200_BATCHER=batching`` for arrival-time batches), which groups concurrent pages
-into one ``generate`` call -- the role continuous batching plays inside the vLLM server.  Decoding is greedy
-(BASELINE.json); ``temperature`` / ``top_p`` are accepted and ignored.  Standard library only: no web framework.
+into one ``generate`` call -- the role continuous batching plays inside the vLLM server.
+
+Sampling (``--sampling``, default: environment ``DOTS_B200_SAMPLING``, else ``greedy``):
+  * ``greedy``   every page decodes greedily (BASELINE.json); ``temperature`` / ``top_p`` / ``top_k`` / ``seed`` are accepted
+                 and ignored;
+  * ``request``  each request's ``temperature``, ``top_p``, ``seed`` (OpenAI fields) and ``top_k`` (vLLM's ``extra_body``
+                 field; -1 or 0 = off) are honoured, missing ones taking OpenAI's defaults (1.0, 1.0, off, a random seed);
+                 malformed or out-of-range values are a 400.
+Standard library only: no web framework.
 """
 from __future__ import annotations
 
@@ -105,6 +112,27 @@ def parse_chat_request(body: dict) -> Tuple[object, str, int]:
     return images[0], prompt, n
 
 
+def parse_sampling(body: dict):
+    """``SamplingParams`` out of a chat.completions request (``request`` policy), or BadRequest.  A missing seed is drawn
+    here, when the request arrives."""
+    from .sampling import SamplingParams
+
+    def num(name, default, kind):
+        v = body.get(name)
+        if v is None:
+            return default
+        if isinstance(v, bool) or not isinstance(v, (int, float)) or (kind is int and not float(v).is_integer()):
+            raise BadRequest(f"{name} must be {'an integer' if kind is int else 'a number'}, got {v!r}")
+        return kind(v)
+
+    top_k = num("top_k", 0, int)
+    try:
+        return SamplingParams(temperature=num("temperature", 1.0, float), top_p=num("top_p", 1.0, float),
+                              top_k=0 if top_k == -1 else top_k, seed=num("seed", None, int)).with_seed()
+    except ValueError as e:
+        raise BadRequest(str(e)) from None
+
+
 class _Handler(BaseHTTPRequestHandler):
     protocol_version = "HTTP/1.1"
     server_version = "dots_ocr_b200"
@@ -112,6 +140,7 @@ class _Handler(BaseHTTPRequestHandler):
     # set by make_server
     runner = None
     model_name = "rednote-hilab/dots.mocr"
+    sampling = "greedy"
     _ids = itertools.count(1)
     quiet = True
 
@@ -152,14 +181,18 @@ class _Handler(BaseHTTPRequestHandler):
         raw = self.rfile.read(length)
         if path != "/v1/chat/completions":
             return self._error(404, f"no route {self.path}", "not_found_error")
+        kw = {}
         try:
-            image, prompt, n_new = parse_chat_request(json.loads(raw.decode("utf-8")))
+            body = json.loads(raw.decode("utf-8"))
+            image, prompt, n_new = parse_chat_request(body)
+            if self.sampling == "request":
+                kw["sampling"] = parse_sampling(body)
         except BadRequest as e:
             return self._error(400, str(e), "invalid_request_error")
         except (UnicodeDecodeError, json.JSONDecodeError) as e:
             return self._error(400, f"body is not JSON: {e}", "invalid_request_error")
         try:
-            text = self.runner.infer(image, prompt, max_new_tokens=n_new)
+            text = self.runner.infer(image, prompt, max_new_tokens=n_new, **kw)
         except Exception as e:          # engine / kernel errors: the client sees a 500 with the message
             return self._error(500, f"{type(e).__name__}: {e}", "server_error")
         self._send(200, {
@@ -171,10 +204,15 @@ class _Handler(BaseHTTPRequestHandler):
 
 
 def make_server(runner, host: str = "127.0.0.1", port: int = 8000, model_name: str = "rednote-hilab/dots.mocr",
-                quiet: bool = True) -> ThreadingHTTPServer:
-    """A ready (not yet serving) HTTP server around ``runner`` (anything with ``infer(image, prompt, max_new_tokens)``).
-    ``port=0`` picks a free port (``server.server_address[1]``)."""
-    handler = type("DotsHandler", (_Handler,), dict(runner=runner, model_name=model_name, quiet=quiet))
+                quiet: bool = True, sampling: Optional[str] = None) -> ThreadingHTTPServer:
+    """A ready (not yet serving) HTTP server around ``runner`` (anything with ``infer(image, prompt, max_new_tokens)``;
+    under ``sampling="request"`` also taking ``sampling=``).  ``port=0`` picks a free port (``server.server_address[1]``).
+    ``sampling``: ``greedy`` or ``request`` (default: ``dots_ocr_b200.sampling.sampling_policy()``)."""
+    from .sampling import POLICIES, sampling_policy
+    sampling = sampling or sampling_policy()
+    if sampling not in POLICIES:
+        raise ValueError(f"sampling must be one of {POLICIES}, got {sampling!r}")
+    handler = type("DotsHandler", (_Handler,), dict(runner=runner, model_name=model_name, quiet=quiet, sampling=sampling))
     srv = ThreadingHTTPServer((host, port), handler)
     srv.daemon_threads = True
     return srv
@@ -196,8 +234,13 @@ def main(argv: Optional[list] = None) -> None:
     ap.add_argument("--weights-dir", default="./weights/DotsOCR")
     ap.add_argument("--max-batch", type=int, default=64)
     ap.add_argument("--gpus", type=int, default=1, help="worker processes, one per GPU (cuda:0..N-1); pages go to the least-loaded")
+    ap.add_argument("--sampling", choices=["greedy", "request"], default=None,
+                    help="greedy: ignore the requests' sampling fields; request: honour temperature / top_p / top_k / seed "
+                         "(default: $DOTS_B200_SAMPLING, else greedy)")
     ap.add_argument("--verbose", action="store_true")
     a = ap.parse_args(argv)
+    from .sampling import sampling_policy
+    sampling = a.sampling or sampling_policy()
     if a.gpus > 1:
         from .multigpu import MultiGpuRunner, b200_worker
         runner = MultiGpuRunner(a.gpus, factory=b200_worker, factory_args=(a.weights_dir, None, a.max_batch))
@@ -205,8 +248,8 @@ def main(argv: Optional[list] = None) -> None:
         from .continuous import serving_front
         from .runner import PageRunner
         runner = serving_front(PageRunner.from_default(device=a.device, weights_dir=a.weights_dir), max_batch=a.max_batch)
-    srv = make_server(runner, a.host, a.port, a.model_name, quiet=not a.verbose)
-    print(f"dots_ocr_b200 serving {a.model_name} on http://{a.host}:{srv.server_address[1]}/v1", flush=True)
+    srv = make_server(runner, a.host, a.port, a.model_name, quiet=not a.verbose, sampling=sampling)
+    print(f"dots_ocr_b200 serving {a.model_name} on http://{a.host}:{srv.server_address[1]}/v1 ({sampling} decoding)", flush=True)
     try:
         srv.serve_forever()
     except KeyboardInterrupt:

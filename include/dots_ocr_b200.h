@@ -210,6 +210,20 @@ DOTS_API int dots_argmax_advance(const void* logits, long long ldl, int batch, i
                         const long long* stop_ids, int n_stops, long long pad_id, const long long* forced_ids,
                         long long forced_ld, void* stream);
 
+/* Sampled step with per-row parameters, then the bookkeeping of dots_argmax_advance (same arguments, same nullability).
+ * temperature[batch] (f32), top_p[batch] (f32), top_k[batch] (i32), seed[batch] (u64) are DEVICE arrays, read at run time
+ * (a captured decode graph picks up rewritten values).  Per row, on the logits in fp32, in HF's warper order:
+ * temperature < 1e-5 -> greedy, bit-identical to dots_argmax_advance; top_k > 0 keeps l >= the k-th largest l (ties kept);
+ * top_p < 1 keeps, among those, every l whose softmax(l / T) mass of strictly larger logits is < top_p (ties with the last
+ * kept value kept); the token is argmax over the kept set of l / T - log(-log u), u from Philox4x32-10 with key = seed[b]
+ * and counter = (index >> 2, step[b], 0, 0), word index & 3, u = ((x >> 8) + 0.5) * 2^-24.  A row's token depends only on
+ * its logits, parameters, seed and step. */
+DOTS_API int dots_sample_advance(const void* logits, long long ldl, int batch, int vocab, long long* next_ids,
+                        long long* out_ids, long long out_ld, int* step, int* pos, int* ctx_len, int* finished,
+                        const long long* stop_ids, int n_stops, long long pad_id, const long long* forced_ids,
+                        long long forced_ld, const float* temperature, const float* top_p, const int* top_k,
+                        const unsigned long long* seed, void* stream);
+
 /* ---- decode-step fused finalize kernels (split-K reduce + HF rounding points) ------------------ */
 /* First kernel of a decode step: resid = embed[ids]; normed = RMSNorm(resid) * w; also zeroes counters[0..n_counters) -- the
  * rendezvous counters of this step's dots_decode_gemm_resnorm launches (counters may be NULL with n_counters == 0).
